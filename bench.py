@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun, one rank per GPU)
   python bench.py --impl reference ...                      (CPU baseline arm: the oracle port on host cores)
+  python bench.py ... --dump-outputs DIR                    (also write the last timed step's note events as .npy)
 
 Workload (BASELINE.json configs[3], the configuration the 1/2/4/8-GPU metric is quoted on): 10 s synthetic
 22 050 Hz clips (every clip its own seed), full pipeline to note events, sharded by file with no data-path
@@ -260,6 +261,47 @@ def parity_report(model, clips, sample_idx, threads: int):
     }  # fmt: skip
 
 
+DUMP_BYTES = 64 << 20  # cap of --dump-outputs
+
+
+def dump_outputs(dump_dir: str, out) -> None:
+    """Write what bp_transcribe_device returned to its caller in the last timed step as dump_dir/<name>.npy: per clip
+    `frame_off` and `note_off`, per note `start_frame`, `end_frame`, `pitch_midi`, `amplitude` and `bend_off`, and the
+    flat `bends` (offsets as float64, the rest as float32; every integer is exact).  The clips are seeded, so two builds
+    given the same arguments can be compared array by array.  Past DUMP_BYTES a fixed seeded sample of whole clips is
+    written instead; `clip_index` lists the clips written."""
+    a, n_files = out.a, out.n_files
+    note_off = a["note_off"][: n_files + 1].astype(np.int64)
+    frame_off = a["frame_off"][: n_files + 1].astype(np.int64)
+    bend_off = a["bend_off"][: note_off[-1] + 1].astype(np.int64)
+    clip_bends = bend_off[note_off]  # bends of clip i: clip_bends[i] .. clip_bends[i + 1]
+    cost = 24 + 24 * np.diff(note_off) + 4 * np.diff(clip_bends)  # bytes per clip in the files below
+    clips = np.arange(n_files)
+    budget = DUMP_BYTES - 4096  # .npy headers and the leading zero of each offset array
+    if cost.sum() > budget:
+        order = np.random.default_rng(0).permutation(n_files)
+        clips = np.sort(order[np.cumsum(cost[order]) <= budget])
+    notes = np.concatenate([np.arange(note_off[i], note_off[i + 1]) for i in clips] + [np.zeros(0, np.int64)])
+
+    def rebase(counts):
+        return np.concatenate([[0], np.cumsum(counts)]).astype(np.float64)
+
+    arrays = {
+        "clip_index": clips.astype(np.float64),
+        "frame_off": rebase(np.diff(frame_off)[clips]),
+        "note_off": rebase(np.diff(note_off)[clips]),
+        "start_frame": a["start"][notes].astype(np.float32),
+        "end_frame": a["end"][notes].astype(np.float32),
+        "pitch_midi": a["pitch"][notes].astype(np.float32),
+        "amplitude": a["amp"][notes].astype(np.float32),
+        "bend_off": rebase(np.diff(bend_off)[notes]),
+        "bends": np.concatenate([a["bends"][clip_bends[i] : clip_bends[i + 1]] for i in clips] + [np.zeros(0, np.int32)]).astype(np.float32),
+    }
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(dump_dir, f"{name}.npy"), arr)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -270,6 +312,8 @@ def main():
     ap.add_argument("--cpu-clips", type=int, default=2 * CPU_GROUP, help="clips of the cpu_baseline sample")
     ap.add_argument("--parity-clips", type=int, default=6, help="clips of the step checked against the oracle")
     ap.add_argument("--python-steps", type=int, default=2, help="timed predict_batch() passes for e2e_python")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the note events of the last timed step to DIR/<name>.npy "
+                    "(DIR/rank<r>/ per rank when several ranks run)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -337,6 +381,8 @@ def main():
     ms = timed(dev_step, args.steps)
     launches = model.launch_count - l0
     n_notes = out.n_notes()
+    if args.dump_outputs:  # before the e2e leg reuses `out`
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"), out)
     for _ in range(2):
         host_step()
     ms_e2e = timed(host_step, args.steps)

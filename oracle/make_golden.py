@@ -1,19 +1,21 @@
 #!/usr/bin/env python
 """ORACLE tooling — generate tests/golden/*.npz by running the UNMODIFIED reference modules.
 
-Runs only in the build container (needs /root/reference).  The reference's third-party imports are
+Needs a checkout of the reference project (basic-pitch).  The reference's third-party imports are
 satisfied by oracle/ref_shims (librosa / pretty_midi / mir_eval / resampy stand-ins, and an
 `onnxruntime` stand-in whose arithmetic is oracle/model_ref.py), so every line of the reference's
 `inference.py` host logic and `note_creation.py` decode executes as shipped.
 
-    python oracle/make_golden.py            # rewrites tests/golden/*.npz
+    python oracle/make_golden.py REFERENCE_CHECKOUT     # rewrites tests/golden/
 
-Fixtures written (all small, committed):
+Fixtures written (all committed, every file < 1 MB):
   vocadito10_pcm44k.npz the same clip as stored in the reference's test resources (44.1 kHz int16 mono): ingest tests
-  vocadito10.npz        reference golden posteriorgrams/events (tests/resources/vocadito_10/*.npz),
-                        the 22 050 Hz audio they are checked with, and the events the reference
-                        decode emits for the golden posteriorgrams under several parameter sets
-  decode_cases.npz      posteriorgram inputs (uint16-quantised) + reference decode outputs
+  vocadito10.npz        reference golden note/onset posteriorgrams and events (tests/resources/vocadito_10/*.npz),
+                        the events the reference decode emits for the golden posteriorgrams under several
+                        parameter sets, and every 64th sample of the 22 050 Hz audio they are checked with
+                        (the tests rebuild that audio from vocadito10_pcm44k.npz)
+  vocadito10_contour.npz  reference golden contour posteriorgram
+  decode_cases/*.npz    posteriorgram inputs (uint16-quantised) + reference decode outputs, one file per group
   host_cases.npz        window counts / unwrap lengths from the reference's windowing code
   predict_2s.npz        config-1 clip: int16 audio + reference predict() outputs (fake-ORT oracle model)
 """
@@ -21,12 +23,15 @@ import hashlib
 import io
 import pathlib
 import sys
+import tempfile
 import warnings
 
 import numpy as np
 
 ROOT = pathlib.Path(__file__).resolve().parent.parent
-REF = pathlib.Path("/root/reference")
+if len(sys.argv) != 2:
+    sys.exit(__doc__)
+REF = pathlib.Path(sys.argv[1]).resolve()
 sys.path[:0] = [str(ROOT / "oracle" / "ref_shims"), str(REF), str(ROOT)]
 
 import basic_pitch  # noqa: E402  (the reference package)
@@ -174,10 +179,9 @@ def main() -> None:
         print(f"reference predict() via oracle model vs golden {k}: max-abs {np.abs(out[k] - gold_out[k]).max():.3e}")
     print(f"events: reference-run {len(events)}  golden {len(gold_ev)}")
     store = {
-        "audio22k": audio22k.astype(np.float32),
+        "audio22k_every64": audio22k.astype(np.float32)[::64].copy(),
         "gold_note": gold_out["note"].astype(np.float32),
         "gold_onset": gold_out["onset"].astype(np.float32),
-        "gold_contour": gold_out["contour"].astype(np.float32),
     }
     for k, v in pack_events([tuple(r) for r in gold_ev]).items():
         store[f"gold_events/{k}"] = v
@@ -190,6 +194,7 @@ def main() -> None:
     assert np.array_equal(store["decode0/pitch"], store["gold_events/pitch"])
     assert np.array_equal(store["decode0/bend_flat"], store["gold_events/bend_flat"])
     np.savez_compressed(GOLD / "vocadito10.npz", **store)
+    np.savez_compressed(GOLD / "vocadito10_contour.npz", gold_contour=gold_out["contour"].astype(np.float32))
     # the clip as stored (44.1 kHz, 16-bit mono): input of the device ingest tests (csrc/ingest.cu)
     from scipy.io import wavfile
 
@@ -247,8 +252,13 @@ def main() -> None:
             "contour": smooth_fuzz(rng, n_t, 264, 3.0),
         }
         add_post(f"tiny{n_t}", post, [dict(), dict(onset_thresh=0.0, frame_thresh=0.05, min_note_len=1)])
-    store["names"] = np.array(names)
-    np.savez_compressed(GOLD / "decode_cases.npz", **store)
+    (GOLD / "decode_cases").mkdir(exist_ok=True)
+    groups = {"notes10s": ("notes10s",), "chords4s": ("chords4s",), "fuzz": ("fuzz0", "fuzz1", "fuzz2"),
+              "short": ("constant", "tiny1", "tiny2", "tiny3", "tiny12", "tiny13", "tiny25")}
+    for group, bases in groups.items():  # tests/golden_util.DECODE_CASE_GROUPS
+        part = {k: v for k, v in store.items() if k.split("/")[0] in bases}
+        part["names"] = np.array([n for n in names if n.split("/")[0] in bases])
+        np.savez_compressed(GOLD / "decode_cases" / f"{group}.npz", **part)
 
     # ---------------------------------------------------------------- C. host logic
     lens = [1, 3840, 36163, 36164, 36165, 40004, 44100, 72328, 72329, 200607, 220500, 3969000]
@@ -280,16 +290,17 @@ def main() -> None:
 
     clip = synth.tones_clip(2.0, seed=0)
     pcm = np.clip(np.round(clip * 32767.0), -32768, 32767).astype(np.int16)
-    tmp = pathlib.Path("/tmp/bp_cfg1.wav")
-    wavfile.write(tmp, 22050, pcm)
-    out, _midi, events = ref_inf.predict(str(tmp), model)
+    with tempfile.TemporaryDirectory() as tmp:
+        wav = pathlib.Path(tmp) / "cfg1.wav"
+        wavfile.write(wav, 22050, pcm)
+        out, _midi, events = ref_inf.predict(str(wav), model)
     store = {"pcm16": pcm, "note": out["note"], "onset": out["onset"], "contour": out["contour"]}
     for k, v in pack_events(events).items():
         store[f"events/{k}"] = v
     print(f"config-1 clip: {out['note'].shape[0]} frames, {len(events)} events")
     np.savez_compressed(GOLD / "predict_2s.npz", **store)
 
-    for f in sorted(GOLD.glob("*.npz")):
+    for f in sorted(GOLD.glob("**/*.npz")):
         print(f"{f.name}: {f.stat().st_size} B")
 
 

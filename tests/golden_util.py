@@ -1,9 +1,38 @@
 """Helpers to read the fixtures written by oracle/make_golden.py."""
 import numpy as np
 
+# tests/golden/decode_cases/<group>.npz: one file per group of posteriorgram inputs (every fixture file stays < 1 MB)
+DECODE_CASE_GROUPS = ("notes10s", "chords4s", "fuzz", "short")
+
 
 def dequant(q):
     return q.astype(np.float32) / np.float32(65535.0)
+
+
+def load_vocadito(golden_dir):
+    """The vocadito fixture as one mapping: vocadito10.npz, the golden contour posteriorgram (vocadito10_contour.npz)
+    and `audio22k`, the 44.1 kHz clip of vocadito10_pcm44k.npz through the package's host resampler — the same
+    samples the reference's golden posteriorgrams were reproduced from, pinned by a stored sample of them."""
+    from basic_pitch_b200 import audio_io
+
+    z = dict(np.load(golden_dir / "vocadito10.npz"))
+    z.update(np.load(golden_dir / "vocadito10_contour.npz"))
+    pcm = np.load(golden_dir / "vocadito10_pcm44k.npz")
+    audio = audio_io.resample(pcm["pcm"].astype(np.float32) / np.float32(32768.0), int(pcm["sample_rate"]))
+    np.testing.assert_array_equal(audio[::64], z.pop("audio22k_every64"), err_msg="host resampler drifted from the fixture")
+    z["audio22k"] = audio
+    return z
+
+
+def load_decode_cases(golden_dir):
+    """Every decode case of tests/golden/decode_cases/ as one mapping; "names" lists the cases."""
+    cases, names = {}, []
+    for group in DECODE_CASE_GROUPS:
+        with np.load(golden_dir / "decode_cases" / f"{group}.npz") as z:
+            names += [str(n) for n in z["names"]]
+            cases.update((k, z[k]) for k in z.files if k != "names")
+    cases["names"] = np.array(names)
+    return cases
 
 
 def case_params(z, name):

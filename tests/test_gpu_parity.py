@@ -10,7 +10,8 @@ import pathlib
 import numpy as np
 import pytest
 
-from tests.golden_util import assert_events_equal, case_expected, case_params, dequant, events_to_arrays
+from tests.golden_util import (assert_events_equal, case_expected, case_params, dequant, events_to_arrays,
+                               load_decode_cases, load_vocadito)
 
 pytestmark = pytest.mark.gpu
 ROOT = pathlib.Path(__file__).resolve().parents[1]
@@ -125,7 +126,7 @@ def test_vocadito_golden_posteriorgrams(model, golden_dir, weights_np):
     """reference: tests/test_inference.py:43-70 — shapes, and values vs the golden npz."""
     from oracle import host_ref, model_ref
 
-    z = np.load(golden_dir / "vocadito10.npz")
+    z = load_vocadito(golden_dir)
     audio = z["audio22k"]
     out = model.run_inference_arrays([audio])[0]
     o = model_ref.forward(host_ref.window_audio(audio), weights_np)
@@ -151,7 +152,7 @@ def _gpu_decode(model, post, p):
 
 def test_decode_reference_golden_events(model, golden_dir):
     """reference: tests/test_inference.py:72-76 — the 28 golden events from the golden posteriorgrams."""
-    z = np.load(golden_dir / "vocadito10.npz")
+    z = load_vocadito(golden_dir)
     post = {k: z[f"gold_{k}"] for k in ("note", "onset", "contour")}
     got = _gpu_decode(model, post, dict(onset_thresh=0.5, frame_thresh=0.3, min_note_len=11, infer_onsets=True,
                                         melodia_trick=True, min_freq=None, max_freq=None))
@@ -166,7 +167,7 @@ def test_decode_reference_golden_events(model, golden_dir):
 
 @pytest.mark.parametrize("i", range(9))
 def test_decode_bit_exact_vocadito_param_sets(model, golden_dir, i):
-    z = np.load(golden_dir / "vocadito10.npz")
+    z = load_vocadito(golden_dir)
     post = {k: z[f"gold_{k}"] for k in ("note", "onset", "contour")}
     got = _gpu_decode(model, post, case_params(z, f"decode{i}"))
     assert_events_equal(got, case_expected(z, f"decode{i}"), ctx=f"decode{i}")
@@ -175,7 +176,7 @@ def test_decode_bit_exact_vocadito_param_sets(model, golden_dir, i):
 def test_decode_bit_exact_reference_cases(model, golden_dir):
     """Every case produced by the UNMODIFIED reference decode: dense chords, fuzz, thresholds <= 0,
     NaN path (constant input), 1..25-frame inputs, frequency limits, melodia on/off."""
-    z = np.load(golden_dir / "decode_cases.npz")
+    z = load_decode_cases(golden_dir)
     for name in z["names"]:
         name = str(name)
         base = name.rsplit("/", 1)[0]
@@ -186,7 +187,7 @@ def test_decode_bit_exact_reference_cases(model, golden_dir):
 
 def test_decode_batch_equals_single(model, golden_dir):
     """Files decoded in one batched call give the same events as one call per file (incl. an empty file)."""
-    z = np.load(golden_dir / "decode_cases.npz")
+    z = load_decode_cases(golden_dir)
     bases = ["notes10s", "fuzz0", "tiny3", "chords4s", "constant"]
     posts = [{k: dequant(z[f"{b}/{k}_q"]) for k in ("note", "onset", "contour")} for b in bases]
     posts.insert(2, {"note": np.zeros((0, 88), np.float32), "onset": np.zeros((0, 88), np.float32), "contour": np.zeros((0, 264), np.float32)})
@@ -555,7 +556,7 @@ def test_device_ingest_vocadito_44k_vs_golden(model, golden_dir):
     lib = model._lib
     audio = np.empty(int(lib.bp_resampled_length(len(pcm), sr)), np.float32)
     lib.bp_load_pcm_host(model.handle, pcm.ctypes.data, 1, len(pcm), 1, sr, audio.ctypes.data)
-    gold = np.load(golden_dir / "vocadito10.npz")
+    gold = load_vocadito(golden_dir)
     assert np.abs(audio - gold["audio22k"]).max() < 3e-6  # the host resampler of the fixture
     out = model.run_inference_arrays([audio])[0]
     for k in ("note", "onset", "contour"):

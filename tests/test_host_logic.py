@@ -3,6 +3,7 @@ import numpy as np
 import pytest
 
 from oracle import decode_ref
+from tests.golden_util import load_vocadito
 
 
 def test_weight_blob_roundtrip_and_dsp_constants(weights_np):
@@ -249,7 +250,7 @@ def test_window_audio_file_and_get_audio_input_like_the_reference_tests(golden_d
     from basic_pitch_b200 import inference as inf
     from basic_pitch_b200.constants import AUDIO_N_SAMPLES, AUDIO_SAMPLE_RATE, FFT_HOP
 
-    audio = np.load(golden_dir / "vocadito10.npz")["audio22k"]
+    audio = load_vocadito(golden_dir)["audio22k"]
     windows, times = zip(*inf.window_audio_file(audio, AUDIO_N_SAMPLES - 30 * FFT_HOP))
     assert len(windows) == 6 and len(times) == 6
     assert all(t["start"] <= t["end"] for t in times)

@@ -4,14 +4,15 @@ import numpy as np
 import pytest
 
 from oracle import decode_ref, host_ref, model_ref
-from tests.golden_util import assert_events_equal, case_expected, case_params, dequant, events_to_arrays
+from tests.golden_util import (assert_events_equal, case_expected, case_params, dequant, events_to_arrays,
+                               load_decode_cases, load_vocadito)
 
 
 def test_model_restatement_vs_reference_golden(golden_dir, weights_np):
     """reference: tests/test_inference.py:66-70 checks every runtime against this vector at atol=1e-4.
     Here the 44.1 kHz -> 22.05 kHz resampler differs from librosa's soxr_hq, which costs ~2e-4
     (measured 4.6e-5 / 2.1e-4 / 1.1e-4); tolerance 5e-4."""
-    z = np.load(golden_dir / "vocadito10.npz")
+    z = load_vocadito(golden_dir)
     audio = z["audio22k"]
     assert audio.shape[0] == 200607  # reference: tests/test_inference.py:194
     win = host_ref.window_audio(audio)
@@ -27,7 +28,7 @@ def test_model_restatement_vs_reference_golden(golden_dir, weights_np):
 def test_model_restatement_f32_vs_f64(golden_dir, weights_np):
     import torch
 
-    z = np.load(golden_dir / "vocadito10.npz")
+    z = load_vocadito(golden_dir)
     win = host_ref.window_audio(z["audio22k"])[:2]
     a = model_ref.forward(win, weights_np, torch.float32)
     b = model_ref.forward(win, weights_np, torch.float64)
@@ -53,7 +54,7 @@ def _run_decode(post, params):
 
 def test_decode_restatement_vs_reference_golden_events(golden_dir):
     """reference: tests/test_inference.py:72-76 (28 golden events)."""
-    z = np.load(golden_dir / "vocadito10.npz")
+    z = load_vocadito(golden_dir)
     post = {k: z[f"gold_{k}"] for k in ("note", "onset", "contour")}
     got = _run_decode(post, dict(onset_thresh=0.5, frame_thresh=0.3, min_note_len=11, infer_onsets=True,
                                  melodia_trick=True, min_freq=None, max_freq=None))
@@ -68,14 +69,14 @@ def test_decode_restatement_vs_reference_golden_events(golden_dir):
 
 @pytest.mark.parametrize("i", range(9))
 def test_decode_restatement_vs_reference_run_vocadito(golden_dir, i):
-    z = np.load(golden_dir / "vocadito10.npz")
+    z = load_vocadito(golden_dir)
     post = {k: z[f"gold_{k}"] for k in ("note", "onset", "contour")}
     got = _run_decode(post, case_params(z, f"decode{i}"))
     assert_events_equal(got, case_expected(z, f"decode{i}"), ctx=f"decode{i}")
 
 
 def test_decode_restatement_vs_reference_run_cases(golden_dir):
-    z = np.load(golden_dir / "decode_cases.npz")
+    z = load_decode_cases(golden_dir)
     for name in z["names"]:
         name = str(name)
         base = name.rsplit("/", 1)[0]
