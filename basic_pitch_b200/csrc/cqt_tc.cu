@@ -10,21 +10,26 @@
 // (`get_cqt_complex`, reflect pad + two strided conv1d per octave), :642-661 (concat, sqrt(len) scaling, magnitude) and
 // layers/signal.py:174-176 (power -> 10*log10(. + 1e-10)); the per-window min / max feed lognorm_kernel (hcqt.cu).
 //
-// Two kernels compute it: cqt_ts_kernel (default, further down: A operand written to TENSOR memory by the producers,
-// TS-form MMAs) and cqt_tc_kernel (BP_B200_CQT_SS=1: A operand staged in shared memory, described next).
-//
 // The A operand is an overlapping strided view of the signal (row t starts at sample t*hop), which no UMMA/TMA
-// descriptor can express for hop*4 B < 16 B or non-canonical pitches, so it is staged explicitly ("im2col" into the
-// canonical K-major core-matrix layout) by four producer warps that also do the reflect padding and the hi/lo split.
+// descriptor can express for hop*4 B < 16 B or non-canonical pitches, so producer warps build it explicitly (reflect
+// padding and three-way split included) and write it to TENSOR memory, where TS-form MMAs read it.  A producer lane owns
+// one frame row: it loads its 16 taps of the chunk (global memory through L1: the rows of an item overlap, the lines stay
+// hot), splits them three ways in registers and writes them with tcgen05.st straight into the tensor-memory columns the
+// MMAs read (kind::f16 A-in-TMEM layout: row = lane, two bf16 per column, K = 16 -> 8 columns; 3 planes x 32 columns per
+// chunk).  No operand tile in shared memory, so the whole split kernel matrix (120 KB) stays resident instead of being
+// streamed per chunk.  Shared-memory traffic per chunk: 60 KB of B reads.
 //
 // item = (M-tile of 128 frames, octave); per item 4 K-chunks of 64 taps, each chunk = 4 k-steps x 6 products:
-//   warps 8-23  producers: gather 128 x 64 samples (128-bit loads where aligned), split, st.shared into
-//               [plane][k/8][row][8] ; one lane bulk-copies the matching 30 KB slice of the split kernel matrix W
-//               (UBLKCP) ; fence.proxy.async ; mbarrier arrive
-//   warp 24     MMA issuer (one elected lane): 24 tcgen05.mma per chunk, tcgen05.commit frees the stage / publishes TMEM
-//   warps 0-7   epilogue (two per TMEM lane quadrant): tcgen05.ld 32 / 40 columns, magnitude * sqrt(len), log-power, store, per-window min/max (atomics)
-// (the issue arbiter prefers high warp ids: the MMA issuer and the producers, which bound the kernel, outrank the epilogue)
-// Shared memory: 2 stages x (48 KB A + 30 KB W); TMEM: 2 accumulators of 128 x 80 (256 columns allocated).
+//   warps 8-23  producers: warp w serves TMEM lane quadrant w % 4 and the taps 16 (w / 4) .. 16 (w / 4) + 15 of every
+//               chunk (k-step w / 4); tcgen05.st of the three planes, mbarrier arrive
+//   warp 24     MMA issuer (one elected lane): bulk-copies the split kernel matrix once per CTA, then 24 TS-form
+//               tcgen05.mma per chunk; tcgen05.commit frees the A stage / publishes the accumulator
+//   warps 0-7   epilogue (two per TMEM lane quadrant): tcgen05.ld 32 / 40 columns, magnitude * sqrt(len), log-power, store,
+//               per-window min/max (atomics)
+// (the warp scheduler prefers high warp ids when it picks the next instruction: the MMA issuer and the producers
+// outrank the epilogue)
+// Shared memory: the split kernel matrix + the epilogue's staging tiles; tensor memory: 3 A stages x 96 columns at
+// 0 / 96 / 192, accumulators (80 columns) at 288 and 416.
 #include <cuda_bf16.h>
 
 #include <cstdio>
@@ -40,23 +45,22 @@ namespace cq {
 constexpr int kMTile = 128;
 constexpr int kKc = 64;                          // taps per chunk
 constexpr int kN = 80;                           // 72 columns padded to a multiple of 16
-constexpr int kAPlane = (kKc / 8) * kMTile * 16;  // 16384 B : [8 k-chunks of 8][128 rows][16 B]
-constexpr int kWPlane = (kKc / 8) * kN * 16;      // 10240 B : [8][80][16 B]
-constexpr int kStageBytes = 3 * kAPlane + 3 * kWPlane;  // 79872
-constexpr int kStages = 2;
-constexpr int kRowsPerWarp = 8;   // rows of the M-tile a producer warp gathers and converts
-constexpr int kProducers = 32 * kMTile / kRowsPerWarp;  // 16 producer warps (more warps in flight hide the gather latency)
+constexpr int kWPlane = (kKc / 8) * kN * 16;      // 10240 B : [8 k-chunks of 8][80][16 B]
+constexpr int kWBytes = 4 * 3 * kWPlane;          // 122 880: the whole split kernel matrix
+constexpr int kProducers = 4 * (kKc / 16) * 32;   // 4 TMEM lane quadrants x 4 k-steps x 32 lanes (rows): 16 producer warps
+static_assert(kProducers == 512, "producer geometry");
 constexpr int kEpiWarps = 8;                      // two per TMEM lane quadrant: bins 0..15 / 16..35 of the octave
 constexpr int kThreads = kProducers + 32 + 32 * kEpiWarps;
+static_assert(kThreads <= 1024, "block size");
 constexpr int kTilePitch = 21;                    // epilogue staging: [8 warps][32 rows][<= 20 bins + 1]
-constexpr int kStgPitch = 68;                     // producer staging: [128 rows][64 taps + 4] fp32
-constexpr int kSegOctave = 3;                     // octaves >= this (hop <= 32) stage their signal segment once per item
-constexpr int kSegPlane = (kMTile * kStgPitch * 4 / (3 * 2)) & ~7;  // bf16 elements per plane of the segment (5800)
-static_assert(kSegPlane >= 126 * 32 + 2 * kTaps + 32, "segment of the hop-32 octave");
 constexpr int kEpiBytes = kEpiWarps * 32 * kTilePitch * 4;
-constexpr int kSmemBytes = kStages * kStageBytes + 256 + kEpiBytes + kMTile * kStgPitch * 4 + kMTile * 24;
-static_assert(kThreads <= 1024 && kRowsPerWarp % 2 == 0 && (kKc * kRowsPerWarp / 32) % 8 == 0, "producer geometry");
+constexpr int kSmemBytes = kWBytes + kEpiBytes + 256;
+// tensor memory (512 columns)
+constexpr int kStages = 3;                        // A operand stages
+constexpr int kAStageCols = 96;
+constexpr int kAccCol0 = 288, kAccCol1 = 416;  // (+32 stays a multiple of 32 for the epilogue's x32 loads)
 }  // namespace cq
+
 
 static inline uint16_t f2bf_rn(float x) {
   uint32_t u;
@@ -91,11 +95,6 @@ void build_cqt_tc_weights(const float* cqt_real /* [36][256] */, const float* cq
     }
 }
 
-struct RowP {  // where one frame row of the current item reads its signal (producer scratch in shared memory)
-  const float* src;
-  int i0, lo, hi, live;
-};
-
 struct CqtTcArgs {
   const float* audio;
   const WinDesc* desc;   // may be null: window b = audio + b*43844
@@ -114,15 +113,18 @@ struct CqtTcArgs {
 #define CQ_TRACE(i, ev) do { } while (0)
 #endif
 
-__global__ void __launch_bounds__(cq::kThreads, 1) cqt_tc_kernel(const CqtTcArgs a) {
+__global__ void __launch_bounds__(cq::kThreads, 1) cqt_ts_kernel(const CqtTcArgs a) {
   using namespace cq;
   extern __shared__ __align__(128) unsigned char smem[];
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kStages * kStageBytes);
-  uint64_t* full = bars;              // [kStages]  128 producer arrivals + the bytes of the W slice
-  uint64_t* empty = bars + kStages;   // [kStages]
-  uint64_t* tmem_full = bars + 2 * kStages;   // [2]
-  uint64_t* tmem_empty = tmem_full + 2;       // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty + 2);
+  unsigned char* s_w = smem;  // [chunk 4][plane 3][k/8 8][n 80][16 B]
+  float* s_tile = reinterpret_cast<float*>(smem + kWBytes);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kWBytes + kEpiBytes);
+  uint64_t* a_full = bars;                  // [3] 16 producer-warp arrivals
+  uint64_t* a_empty = bars + kStages;       // [3] commit behind the MMAs that read the stage
+  uint64_t* tmem_full = a_empty + kStages;  // [2]
+  uint64_t* tmem_empty = tmem_full + 2;     // [2]
+  uint64_t* w_full = tmem_empty + 2;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(w_full + 1);
 
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);  // broadcast: warp-uniform role branches and loop state
   const int lane = threadIdx.x & 31;
@@ -130,17 +132,18 @@ __global__ void __launch_bounds__(cq::kThreads, 1) cqt_tc_kernel(const CqtTcArgs
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < kStages; ++s) {
-      mbar_init(full + s, kProducers / 32);  // one arrival per producer warp (512 single arrivals per chunk serialise)
-      mbar_init(empty + s, 1);
+      mbar_init(a_full + s, kProducers / 32);
+      mbar_init(a_empty + s, 1);
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(tmem_full + i, 1);
       mbar_init(tmem_empty + i, kEpiWarps);
     }
+    mbar_init(w_full, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == kMmaWarp) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(256));
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512));
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
   tc_fence_before();
@@ -153,266 +156,123 @@ __global__ void __launch_bounds__(cq::kThreads, 1) cqt_tc_kernel(const CqtTcArgs
 
   if (warp >= kEpiWarps && warp < kMmaWarp) {
     // ------------------------------ producers ------------------------------
-    // Phase A (lanes along the taps): warp pw gathers rows RW pw .. RW pw + RW - 1 of the chunk, two rows (2 x 64 taps) per
-    // 128-bit load instruction, into the staging tile S[row][64 taps] -- a load instruction touches 4-6 cache lines
-    // instead of 32 (one per row), which is what the LSU pipe was saturated with.  Phase B (lanes along the rows): thread
-    // (row, half) reads its 32 taps back, splits them three ways and writes the K-major operand tile.
-    constexpr int RW = kRowsPerWarp, NI = RW / 2;  // row pairs per warp
-    constexpr int KQ = 32 / RW;                    // phase B: lanes per row
-    constexpr int TPL = kKc / KQ;                  // taps per lane in phase B (a multiple of 8)
-    const int ptid = threadIdx.x - 32 * kEpiWarps;  // producer thread
-    const int pw = ptid >> 5;
-    const int r = RW * pw + (lane % RW);  // phase B: the warp converts the rows it gathered, no block-wide barrier
-    const int kq = lane / RW;
-    float* stg = reinterpret_cast<float*>(smem + kStages * kStageBytes + 256 + kEpiBytes);  // [128][kStgPitch]
-    RowP* rowp = reinterpret_cast<RowP*>(smem + kStages * kStageBytes + 256 + kEpiBytes +
-                                         kMTile * kStgPitch * 4) + RW * pw;  // this warp's rows
-    uint32_t stage = 0, ph = 0;
+    const int pw = warp - kEpiWarps;
+    const int quad = pw & 3, ks = pw >> 2;  // TMEM lane quadrant; k-step (taps 16 ks .. 16 ks + 15 of every chunk)
+    const int row = quad * 32 + lane;
+    const uint32_t lane_base = tmem_base + ((uint32_t)(quad * 32) << 16);
+    uint32_t g = 0;  // chunks produced so far -> stage g % 3
     int icnt = -1;
     for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
       ++icnt;
+      if (pw == 0) CQ_TRACE(icnt, 0);  // producer warp 0 starts the item
       const int mt = it / kOctaves, o = it % kOctaves;
       const int hop = 256 >> o;
-      if (pw == 0) CQ_TRACE(icnt, 0);  // producer warp 0 starts the item
       const int len = octave_len_rt(o);
-      // The staging area is shared by both paths (rows of a warp / planes of the item's segment): nobody may start
-      // writing it for this item while another producer warp still reads it for the previous one.
-      asm volatile("bar.sync 1, %0;" ::"n"(kProducers) : "memory");
-      if (pw == 0) CQ_TRACE(icnt, 14);  // all producer warps are done with the previous item
-      if (o >= kSegOctave) {
-        // ---- octaves with hop <= 32: the 128 rows of the item overlap (by 7/8 .. 255/256 of their 256 taps), so the signal
-        // segment they cover is loaded, reflect-padded and split three ways ONCE per item into bf16 planes in shared memory
-        // (it fits where the other path stages its rows), and every chunk's operand tile is then assembled with 16-byte
-        // copies: 6 per thread and chunk instead of a gather + split of 16 samples per thread.
-        // An M-tile may span two windows: part 0 = rows [0, n0) (frames t0.. of window b0), part 1 = rows [n0, 128)
-        // (frames 0.. of window b0 + 1).  Each part's segment starts on a multiple of 8 samples at or below its first tap.
-        __nv_bfloat16* seg = reinterpret_cast<__nv_bfloat16*>(stg);
-        const int m0 = mt * kMTile;
-        const int b0 = m0 / kFrames, t0 = m0 - b0 * kFrames;
-        const int n0 = min(kMTile, kFrames - t0);
-        const int s0 = t0 * hop - 128, a0 = s0 & ~7, d0 = s0 - a0;  // part 0: first tap, aligned start, offset of the tap
-        const int L0 = ((n0 - 1) * hop + kTaps + d0 + 7) & ~7;
-        const int L1 = n0 < kMTile ? (((kMTile - n0 - 1) * hop + kTaps + 7) & ~7) : 0;  // part 1 starts at sample -128
-        {
-          // <= 9 samples per thread (126 * 32 + 2 * 256 + slack <= 9 * 512): all loads are issued before the first use
-          constexpr int NS = (126 * 32 + 2 * kTaps + 32 + kProducers - 1) / kProducers;
-          float xs[NS];
-#pragma unroll
-          for (int q = 0; q < NS; ++q) {
-            const int idx = ptid + q * kProducers;
-            const int part = idx >= L0;
-            const int b = b0 + part;
-            int i = part ? idx - L0 - 128 : a0 + idx;
-            if (i < 0) i = -i;
-            if (i >= len) i = 2 * (len - 1) - i;
-            xs[q] = (idx < L0 + L1 && b < a.n_windows && i >= 0 && i < len)
-                        ? __ldg(a.chain + (size_t)b * kChainStride + chain_off_rt(o) + i)
-                        : 0.f;
-          }
-          if (pw == 0 && xs[0] != 123456.f) CQ_TRACE(icnt, 15);  // first load has arrived
-#pragma unroll
-          for (int q = 0; q < NS; ++q) {
-            const int idx = ptid + q * kProducers;
-            if (idx < L0 + L1) {
-              const float x = xs[q];
-              const __nv_bfloat16 h = __float2bfloat16_rn(x);
-              const float r1 = x - __bfloat162float(h);
-              const __nv_bfloat16 md = __float2bfloat16_rn(r1);
-              seg[idx] = h;
-              seg[kSegPlane + idx] = md;
-              seg[2 * kSegPlane + idx] = __float2bfloat16_rn(r1 - __bfloat162float(md));
-            }
-          }
+      const int m = mt * kMTile + row;
+      const bool live = m < total_frames;
+      const int b = live ? m / kFrames : 0;
+      const int t = m - b * kFrames;
+      const float* src;
+      int lo = 0, hi = len;
+      if (o == 0) {
+        if (a.desc) {
+          const WinDesc d = a.desc[b];
+          src = a.audio + d.base;
+          lo = d.lo;
+          hi = d.hi;
+        } else {
+          src = a.audio + (long long)b * kWinSamples;
         }
-        asm volatile("bar.sync 1, %0;" ::"n"(kProducers) : "memory");
-        if (pw == 0) CQ_TRACE(icnt, 1);  // segment staged
-        for (int c = 0; c < kTaps / kKc; ++c) {
-          mbar_wait(empty + stage, ph ^ 1);
-          if (pw == 0) CQ_TRACE(icnt, 2 + c);  // stage acquired for chunk c
-          unsigned char* sa = smem + stage * kStageBytes;
-          if (ptid == 0) {
-            mbar_expect_tx_only(full + stage, 3 * kWPlane);
-            bulk_g2s(sa + 3 * kAPlane, a.wtc + (size_t)c * (3 * kWPlane / 2), 3 * kWPlane, full + stage);
-          }
-#pragma unroll
-          for (int q = 0; q < 3 * 8 * kMTile / kProducers; ++q) {
-            const int id = ptid + q * kProducers;
-            const int row = id & (kMTile - 1), kc = (id >> 7) & 7, pl = id >> 10;
-            const int e = (row < n0 ? d0 + row * hop : L0 + (row - n0) * hop) + c * kKc + kc * 8;  // element inside a plane
-            const __nv_bfloat16* src = seg + pl * kSegPlane + e;
-            uint4 v;
-            if ((e & 7) == 0) {
-              v = *reinterpret_cast<const uint4*>(src);
-            } else if ((e & 1) == 0) {
-              const uint32_t* w = reinterpret_cast<const uint32_t*>(src);
-              v = make_uint4(w[0], w[1], w[2], w[3]);
-            } else {  // odd element offset (hop 1): five words, shifted by half a word
-              const uint32_t* w = reinterpret_cast<const uint32_t*>(src - 1);
-              v = make_uint4(__funnelshift_r(w[0], w[1], 16), __funnelshift_r(w[1], w[2], 16),
-                             __funnelshift_r(w[2], w[3], 16), __funnelshift_r(w[3], w[4], 16));
-            }
-            *reinterpret_cast<uint4*>(sa + pl * kAPlane + (kc * kMTile + row) * 16) = v;
-          }
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-          __syncwarp();
-          if (lane == 0) mbar_arrive(full + stage);
-          if (++stage == kStages) {
-            stage = 0;
-            ph ^= 1;
-          }
-        }
-        continue;
+      } else {
+        src = a.chain + (size_t)b * kChainStride + chain_off_rt(o);
       }
-      __syncwarp();
-      if (lane < RW) {  // per item: where row RW pw + lane reads its signal
-        const int m = mt * kMTile + RW * pw + lane;
-        RowP p;
-        p.live = m < total_frames;
-        const int b = p.live ? m / kFrames : 0;
-        const int t = m - b * kFrames;
-        p.lo = 0;
-        p.hi = len;
-        if (o == 0) {
-          if (a.desc) {
-            const WinDesc d = a.desc[b];
-            p.src = a.audio + d.base;
-            p.lo = d.lo;
-            p.hi = d.hi;
-          } else {
-            p.src = a.audio + (long long)b * kWinSamples;
+      const int i0 = t * hop - 128 + 16 * ks;  // signal index of this lane's first tap in chunk 0
+      auto load16 = [&](int c, float (&x)[16]) {
+        const int ib = i0 + c * kKc;
+        if (live && ib >= max(lo, 0) && ib + 16 <= min(hi, len) && ((reinterpret_cast<uintptr_t>(src + ib) & 15) == 0)) {
+#pragma unroll
+          for (int q = 0; q < 4; ++q) {
+            const float4 v = __ldg(reinterpret_cast<const float4*>(src + ib) + q);
+            x[4 * q] = v.x, x[4 * q + 1] = v.y, x[4 * q + 2] = v.z, x[4 * q + 3] = v.w;
           }
         } else {
-          p.src = a.chain + (size_t)b * kChainStride + chain_off_rt(o);
-        }
-        p.i0 = t * hop - 128;  // signal index of tap 0 of this frame
-        rowp[lane] = p;
-      }
-      __syncwarp();
-      for (int c = 0; c < kTaps / kKc; ++c) {
-        float xs[4 * NI];
-        unsigned vmask = 0;  // row pairs that took the vector path (warp-uniform)
+          // rows at the signal ends (reflect padding, zeros outside [lo, hi)), unaligned low octaves, dead rows
 #pragma unroll
-        for (int i = 0; i < NI; ++i) {
-          // rows 2i, 2i + 1 of the warp's rows; vector path: lane -> (row of the pair, 4 taps)
-          const RowP p = rowp[2 * i + (lane >> 4)];
-          const int ibv = p.i0 + c * kKc;  // signal index of the row's first tap in this chunk
-          const bool okv = p.live && ibv >= p.lo && ibv + kKc <= p.hi && ibv >= 0 && ibv + kKc <= len &&
-                           ((reinterpret_cast<uintptr_t>(p.src + ibv) & 15) == 0);
-          if (__all_sync(0xffffffffu, okv)) {
-            vmask |= 1u << i;
-            const float4 v = __ldg(reinterpret_cast<const float4*>(p.src + ibv) + (lane & 15));
-            xs[4 * i] = v.x, xs[4 * i + 1] = v.y, xs[4 * i + 2] = v.z, xs[4 * i + 3] = v.w;
-          } else {
-            // general path (unaligned low octaves, rows that touch the signal ends): reflect padding, zeros outside
-            // [lo, hi); four loads of (row, 32 consecutive taps)
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              const RowP pq = rowp[2 * i + (q >> 1)];
-              int idx = pq.i0 + c * kKc + (q & 1) * 32 + lane;
-              float xv = 0.f;
-              if (pq.live) {
-                if (idx < 0) idx = -idx;
-                if (idx >= len) idx = 2 * (len - 1) - idx;
-                if (idx >= pq.lo && idx < pq.hi) xv = __ldg(pq.src + idx);
-              }
-              xs[4 * i + q] = xv;
-            }
+          for (int k = 0; k < 16; ++k) {
+            int idx = ib + k;
+            if (idx < 0) idx = -idx;
+            if (idx >= len) idx = 2 * (len - 1) - idx;
+            x[k] = (live && idx >= lo && idx < hi) ? __ldg(src + idx) : 0.f;
           }
         }
-        __syncwarp();  // the warp's staging rows are free (phase B of its previous chunk is done)
+      };
+      float xn[16];
+      load16(0, xn);
+      for (int c = 0; c < kTaps / kKc; ++c, ++g) {
+        float x[16];
 #pragma unroll
-        for (int i = 0; i < NI; ++i) {
-          if ((vmask >> i) & 1u) {  // lanes hold (row of the pair, 4 taps)
-            *reinterpret_cast<float4*>(stg + (RW * pw + 2 * i + (lane >> 4)) * kStgPitch + 4 * (lane & 15)) =
-                make_float4(xs[4 * i], xs[4 * i + 1], xs[4 * i + 2], xs[4 * i + 3]);
-          } else {  // lanes hold 4 x (row, tap)
+        for (int k = 0; k < 16; ++k) x[k] = xn[k];
+        if (c + 1 < kTaps / kKc) load16(c + 1, xn);  // the next chunk's loads are in flight while this one is split and stored
+        uint32_t h[8], md[8], l[8];
 #pragma unroll
-            for (int q = 0; q < 4; ++q)
-              stg[(RW * pw + 2 * i + (q >> 1)) * kStgPitch + (q & 1) * 32 + lane] = xs[4 * i + q];
-          }
+        for (int j = 0; j < 8; ++j) {
+          const __nv_bfloat162 hh = __floats2bfloat162_rn(x[2 * j], x[2 * j + 1]);
+          const float2 hf = __bfloat1622float2(hh);
+          const float r0 = x[2 * j] - hf.x, r1 = x[2 * j + 1] - hf.y;
+          const __nv_bfloat162 mm = __floats2bfloat162_rn(r0, r1);
+          const float2 mf = __bfloat1622float2(mm);
+          const __nv_bfloat162 ll = __floats2bfloat162_rn(r0 - mf.x, r1 - mf.y);
+          h[j] = *reinterpret_cast<const uint32_t*>(&hh);
+          md[j] = *reinterpret_cast<const uint32_t*>(&mm);
+          l[j] = *reinterpret_cast<const uint32_t*>(&ll);
         }
-        __syncwarp();  // rows complete
-        // phase B: this lane's TPL taps of row r
-        float xb[TPL];
-        {
-          const float4* sp = reinterpret_cast<const float4*>(stg + r * kStgPitch + TPL * kq);
-#pragma unroll
-          for (int i = 0; i < TPL / 4; ++i) {
-            const float4 v = sp[i];
-            xb[4 * i] = v.x, xb[4 * i + 1] = v.y, xb[4 * i + 2] = v.z, xb[4 * i + 3] = v.w;
-          }
-        }
-        mbar_wait(empty + stage, ph ^ 1);
-        if (pw == 0) CQ_TRACE(icnt, 2 + c);
-        unsigned char* sa = smem + stage * kStageBytes;
-        if (ptid == 0) {
-          mbar_expect_tx_only(full + stage, 3 * kWPlane);  // the bulk copy of the W slice completes on the same barrier
-          bulk_g2s(sa + 3 * kAPlane, a.wtc + (size_t)c * (3 * kWPlane / 2), 3 * kWPlane, full + stage);
-        }
-#pragma unroll
-        for (int q = 0; q < TPL / 8; ++q) {
-          const int kc = kq * (TPL / 8) + q;
-          const float* x = xb + 8 * q;
-          __align__(16) __nv_bfloat162 h[4], md[4], l[4];
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            h[j] = __floats2bfloat162_rn(x[2 * j], x[2 * j + 1]);
-            const float2 hf = __bfloat1622float2(h[j]);
-            const float r0 = x[2 * j] - hf.x, r1 = x[2 * j + 1] - hf.y;
-            md[j] = __floats2bfloat162_rn(r0, r1);
-            const float2 mf = __bfloat1622float2(md[j]);
-            l[j] = __floats2bfloat162_rn(r0 - mf.x, r1 - mf.y);
-          }
-          const int o16 = (kc * kMTile + r) * 16;
-          *reinterpret_cast<uint4*>(sa + o16) = *reinterpret_cast<const uint4*>(h);
-          *reinterpret_cast<uint4*>(sa + kAPlane + o16) = *reinterpret_cast<const uint4*>(md);
-          *reinterpret_cast<uint4*>(sa + 2 * kAPlane + o16) = *reinterpret_cast<const uint4*>(l);
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> visible to the MMA
+        const uint32_t stage = g % kStages, ph = (g / kStages) & 1u;
+        if (pw == 0) CQ_TRACE(icnt, 14 + (c & 1));  // (c = 2, 3 overwrite: last split done)
+        mbar_wait(a_empty + stage, ph ^ 1u);
+        if (pw == 0) CQ_TRACE(icnt, 2 + c);  // stage acquired for chunk c
+        tc_fence_after();
+        const uint32_t col = lane_base + stage * kAStageCols + (uint32_t)ks * 8u;
+        tmem_st8(col, h);
+        tmem_st8(col + 32, md);
+        tmem_st8(col + 64, l);
+        tmem_st_wait();
+        tc_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive(full + stage);
-        if (++stage == kStages) {
-          stage = 0;
-          ph ^= 1;
-        }
+        if (lane == 0) mbar_arrive(a_full + stage);
       }
     }
   } else if (warp == kMmaWarp) {
-    // ------------------------------ MMA issuer ------------------------------
-    constexpr uint32_t idesc = make_idesc(128, kN);  // kind::f16, bf16 x bf16 -> f32
+    // ------------------------------ MMA issuer (A operand in tensor memory) ------------------------------
+    constexpr uint32_t idesc = make_idesc(128, kN);
     const uint32_t leader = elect_one() ? 1u : 0u;
-    uint32_t stage = 0, ph = 0, icount = 0;
+    // the whole split kernel matrix, once per CTA
+    bulk_g2s_expect_pred(s_w, a.wtc, kWBytes, w_full, leader);
+    const uint32_t desc_hi32 = (128u >> 4) | (1u << 14);
+    const uint32_t w_base = ((smem_u32(s_w) >> 4) & 0x3fffu) | ((uint32_t)(kN * 16 >> 4) << 16);
+    uint32_t g = 0, icount = 0;
     uint32_t ph_t[2] = {0, 0};
+    mbar_wait(w_full, 0);
     for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
       const uint32_t buf = icount & 1u;
       mbar_wait(tmem_empty + buf, ph_t[buf] ^ 1);
       ph_t[buf] ^= 1;
       tc_fence_after();
-      const uint32_t d = tmem_base + buf * 128u;
+      const uint32_t d = tmem_base + (buf ? kAccCol1 : kAccCol0);
       CQ_TRACE(icount, 6);  // accumulator acquired
-      for (int c = 0; c < kTaps / kKc; ++c) {
-        mbar_wait(full + stage, ph);
+      for (int c = 0; c < kTaps / kKc; ++c, ++g) {
+        const uint32_t stage = g % kStages, ph = (g / kStages) & 1u;
+        mbar_wait(a_full + stage, ph);
         CQ_TRACE(icount, 7 + c);  // chunk c's operands arrived
         tc_fence_after();
-        // descriptors as (low word, shared high word); everything here is warp-uniform, the MMAs themselves are
-        // predicated on the elected lane inside the asm block: the loop stays on the uniform datapath (no R2UR per MMA)
-        const uint32_t sa = smem_u32(smem + stage * kStageBytes);
-        const uint32_t desc_hi32 = (128u >> 4) | (1u << 14);
-        const uint32_t a_base = ((sa >> 4) & 0x3fffu) | ((uint32_t)(kMTile * 16 >> 4) << 16);
-        const uint32_t b_base = (((sa + 3 * kAPlane) >> 4) & 0x3fffu) | ((uint32_t)(kN * 16 >> 4) << 16);
+        const uint32_t acol = tmem_base + stage * kAStageCols;
 #pragma unroll
         for (int ks = 0; ks < kKc / 16; ++ks) {
-          // one k-step = 16 taps = two 16-byte k-chunks, LBO apart
-          const uint32_t ao = a_base + (uint32_t)(ks * 2 * (kMTile * 16) >> 4), bo = b_base + (uint32_t)(ks * 2 * (kN * 16) >> 4);
-          umma_bf16_x6(d, ao, ao + (kAPlane >> 4), ao + 2 * (kAPlane >> 4), bo, bo + (kWPlane >> 4), bo + 2 * (kWPlane >> 4),
-                       desc_hi32, idesc, (c | ks) ? 1u : 0u, leader);
+          const uint32_t ah = acol + (uint32_t)ks * 8u;
+          const uint32_t bo = w_base + (uint32_t)(((c * 3) * (kWPlane) + ks * 2 * (kN * 16)) >> 4);
+          umma_ts_bf16_x6(d, ah, ah + 32u, ah + 64u, bo, bo + (kWPlane >> 4), bo + 2 * (kWPlane >> 4), desc_hi32, idesc,
+                          (c | ks) ? 1u : 0u, leader);
         }
-        umma_commit_pred(empty + stage, leader);
-        __syncwarp();
-        if (++stage == kStages) {
-          stage = 0;
-          ph ^= 1;
-        }
+        umma_commit_pred(a_empty + stage, leader);
       }
       umma_commit_pred(tmem_full + buf, leader);
       CQ_TRACE(icount, 11);  // all MMAs of the item issued
@@ -422,13 +282,13 @@ __global__ void __launch_bounds__(cq::kThreads, 1) cqt_tc_kernel(const CqtTcArgs
     // ------------------------------ epilogue (warps 0..7) ------------------------------
     // Two warps per TMEM lane quadrant (a warp may only read lanes 32 (warp % 4) ..): warp < 4 takes bins 0..15 of the
     // octave (accumulator columns 0..31), warp >= 4 bins 16..35 (columns 32..71).  Four warps alone were the bottleneck
-    // of the kernel (busy all the time while the tensor pipe idled at 23 %).
+    // of the kernel (busy all the time while the tensor pipe idled).
     const int quad = warp & 3, half = warp >> 2;
     const int row = quad * 32 + lane;
     const int nb = half ? 20 : 16, bin0 = half ? 16 : 0;
     uint32_t ph_t[2] = {0, 0};
     uint32_t icount = 0;
-    float* tile = reinterpret_cast<float*>(smem + kStages * kStageBytes + 256) + warp * (32 * kTilePitch);
+    float* tile = s_tile + warp * (32 * kTilePitch);
     for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
       const int mt = it / kOctaves, o = it % kOctaves;
       const int m = mt * kMTile + row;
@@ -439,7 +299,7 @@ __global__ void __launch_bounds__(cq::kThreads, 1) cqt_tc_kernel(const CqtTcArgs
       ph_t[buf] ^= 1;
       tc_fence_after();
       if (warp == 0) CQ_TRACE(icount, 12);  // epilogue saw the accumulator
-      const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + buf * 128u + (uint32_t)(2 * bin0);
+      const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (buf ? kAccCol1 : kAccCol0) + (uint32_t)(2 * bin0);
       float vmin = INFINITY, vmax = -INFINITY;
       const int g0 = (8 - o) * kBinsPerOctave - 15 + bin0;  // global bin of this warp's first bin (negative for the lowest of o = 8)
       // 10*log10(re^2 + im^2 + 1e-10) per bin (MUFU.LG2; the reference's sqrt-then-square differs by < 1e-6 dB), staged
@@ -519,291 +379,6 @@ __global__ void __launch_bounds__(cq::kThreads, 1) cqt_tc_kernel(const CqtTcArgs
   tc_fence_before();
   __syncthreads();
   if (warp == kMmaWarp) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256));
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// TS form of the same contraction: the A operand lives in TENSOR memory.
-// cqt_tc_kernel above is bound by shared-memory bandwidth (per 64-tap chunk the producers read and write 48 KB to assemble
-// the operand tile and the SS-mode MMAs read it back three times over).  Here a producer lane owns one frame row: it
-// loads its 16 taps of the chunk (global memory through L1: the rows of an item overlap, the lines stay hot), splits
-// them three ways in registers and writes them with tcgen05.st straight into the tensor-memory columns the MMAs read
-// (kind::f16 A-in-TMEM layout: row = lane, two bf16 per column, K = 16 -> 8 columns; 3 planes x 32 columns per chunk).
-// No operand tile in shared memory, so the whole split kernel matrix (120 KB) stays resident instead of being streamed
-// per chunk.  Shared-memory traffic per chunk: 60 KB of B reads.
-//   warps 0-7   epilogue (unchanged)          warps 8-23  producers: warp w serves TMEM lane quadrant w % 4 and the taps
-//   warp 24     MMA issuer (TS-form)                       16 (w / 4) .. 16 (w / 4) + 15 of every chunk (k-step w / 4)
-// Tensor memory: 3 A stages x 96 columns at 0 / 96 / 192, accumulators (80 columns) at 288 and 416.
-// ------------------------------------------------------------------------------------------------
-namespace cqts {
-constexpr int kStages = 3;
-constexpr int kAStageCols = 96;
-constexpr int kAccCol0 = 288, kAccCol1 = 416;  // (+32 stays a multiple of 32 for the epilogue's x32 loads)
-constexpr int kWBytes = 4 * 3 * cq::kWPlane;  // 122 880: the whole split kernel matrix
-constexpr int kSmemBytes = kWBytes + cq::kEpiBytes + 256;
-}  // namespace cqts
-
-__global__ void __launch_bounds__(cq::kThreads, 1) cqt_ts_kernel(const CqtTcArgs a) {
-  using namespace cq;
-  extern __shared__ __align__(128) unsigned char smem[];
-  unsigned char* s_w = smem;  // [chunk 4][plane 3][k/8 8][n 80][16 B]
-  float* s_tile = reinterpret_cast<float*>(smem + cqts::kWBytes);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + cqts::kWBytes + kEpiBytes);
-  uint64_t* a_full = bars;                     // [3] 16 producer-warp arrivals
-  uint64_t* a_empty = bars + cqts::kStages;    // [3] commit behind the MMAs that read the stage
-  uint64_t* tmem_full = a_empty + cqts::kStages;  // [2]
-  uint64_t* tmem_empty = tmem_full + 2;           // [2]
-  uint64_t* w_full = tmem_empty + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(w_full + 1);
-
-  const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-  const int lane = threadIdx.x & 31;
-  constexpr int kMmaWarp = kEpiWarps + kProducers / 32;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < cqts::kStages; ++s) {
-      mbar_init(a_full + s, kProducers / 32);
-      mbar_init(a_empty + s, 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(tmem_full + i, 1);
-      mbar_init(tmem_empty + i, kEpiWarps);
-    }
-    mbar_init(w_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == kMmaWarp) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  const int n_items = a.n_mtiles * kOctaves;
-  const int total_frames = a.n_windows * kFrames;
-
-  if (warp >= kEpiWarps && warp < kMmaWarp) {
-    // ------------------------------ producers ------------------------------
-    const int pw = warp - kEpiWarps;
-    const int quad = pw & 3, ks = pw >> 2;  // TMEM lane quadrant; k-step (taps 16 ks .. 16 ks + 15 of every chunk)
-    const int row = quad * 32 + lane;
-    const uint32_t lane_base = tmem_base + ((uint32_t)(quad * 32) << 16);
-    uint32_t g = 0;  // chunks produced so far -> stage g % 3
-    int icnt = -1;
-    for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
-      ++icnt;
-      if (pw == 0) CQ_TRACE(icnt, 0);
-      const int mt = it / kOctaves, o = it % kOctaves;
-      const int hop = 256 >> o;
-      const int len = octave_len_rt(o);
-      const int m = mt * kMTile + row;
-      const bool live = m < total_frames;
-      const int b = live ? m / kFrames : 0;
-      const int t = m - b * kFrames;
-      const float* src;
-      int lo = 0, hi = len;
-      if (o == 0) {
-        if (a.desc) {
-          const WinDesc d = a.desc[b];
-          src = a.audio + d.base;
-          lo = d.lo;
-          hi = d.hi;
-        } else {
-          src = a.audio + (long long)b * kWinSamples;
-        }
-      } else {
-        src = a.chain + (size_t)b * kChainStride + chain_off_rt(o);
-      }
-      const int i0 = t * hop - 128 + 16 * ks;  // signal index of this lane's first tap in chunk 0
-      auto load16 = [&](int c, float (&x)[16]) {
-        const int ib = i0 + c * kKc;
-        if (live && ib >= max(lo, 0) && ib + 16 <= min(hi, len) && ((reinterpret_cast<uintptr_t>(src + ib) & 15) == 0)) {
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            const float4 v = __ldg(reinterpret_cast<const float4*>(src + ib) + q);
-            x[4 * q] = v.x, x[4 * q + 1] = v.y, x[4 * q + 2] = v.z, x[4 * q + 3] = v.w;
-          }
-        } else {
-          // rows at the signal ends (reflect padding, zeros outside [lo, hi)), unaligned low octaves, dead rows
-#pragma unroll
-          for (int k = 0; k < 16; ++k) {
-            int idx = ib + k;
-            if (idx < 0) idx = -idx;
-            if (idx >= len) idx = 2 * (len - 1) - idx;
-            x[k] = (live && idx >= lo && idx < hi) ? __ldg(src + idx) : 0.f;
-          }
-        }
-      };
-      float xn[16];
-      load16(0, xn);
-      for (int c = 0; c < kTaps / kKc; ++c, ++g) {
-        float x[16];
-#pragma unroll
-        for (int k = 0; k < 16; ++k) x[k] = xn[k];
-        if (c + 1 < kTaps / kKc) load16(c + 1, xn);  // the next chunk's loads are in flight while this one is split and stored
-        uint32_t h[8], md[8], l[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const __nv_bfloat162 hh = __floats2bfloat162_rn(x[2 * j], x[2 * j + 1]);
-          const float2 hf = __bfloat1622float2(hh);
-          const float r0 = x[2 * j] - hf.x, r1 = x[2 * j + 1] - hf.y;
-          const __nv_bfloat162 mm = __floats2bfloat162_rn(r0, r1);
-          const float2 mf = __bfloat1622float2(mm);
-          const __nv_bfloat162 ll = __floats2bfloat162_rn(r0 - mf.x, r1 - mf.y);
-          h[j] = *reinterpret_cast<const uint32_t*>(&hh);
-          md[j] = *reinterpret_cast<const uint32_t*>(&mm);
-          l[j] = *reinterpret_cast<const uint32_t*>(&ll);
-        }
-        const uint32_t stage = g % cqts::kStages, ph = (g / cqts::kStages) & 1u;
-        if (pw == 0) CQ_TRACE(icnt, 14 + (c & 1));  // (c = 2, 3 overwrite: last split done)
-        mbar_wait(a_empty + stage, ph ^ 1u);
-        if (pw == 0) CQ_TRACE(icnt, 2 + c);
-        tc_fence_after();
-        const uint32_t col = lane_base + stage * cqts::kAStageCols + (uint32_t)ks * 8u;
-        tmem_st8(col, h);
-        tmem_st8(col + 32, md);
-        tmem_st8(col + 64, l);
-        tmem_st_wait();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(a_full + stage);
-      }
-    }
-  } else if (warp == kMmaWarp) {
-    // ------------------------------ MMA issuer (A operand in tensor memory) ------------------------------
-    constexpr uint32_t idesc = make_idesc(128, kN);
-    const uint32_t leader = elect_one() ? 1u : 0u;
-    // the whole split kernel matrix, once per CTA
-    bulk_g2s_expect_pred(s_w, a.wtc, cqts::kWBytes, w_full, leader);
-    const uint32_t desc_hi32 = (128u >> 4) | (1u << 14);
-    const uint32_t w_base = ((smem_u32(s_w) >> 4) & 0x3fffu) | ((uint32_t)(kN * 16 >> 4) << 16);
-    uint32_t g = 0, icount = 0;
-    uint32_t ph_t[2] = {0, 0};
-    mbar_wait(w_full, 0);
-    for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
-      const uint32_t buf = icount & 1u;
-      mbar_wait(tmem_empty + buf, ph_t[buf] ^ 1);
-      ph_t[buf] ^= 1;
-      tc_fence_after();
-      const uint32_t d = tmem_base + (buf ? cqts::kAccCol1 : cqts::kAccCol0);
-      CQ_TRACE(icount, 6);
-      for (int c = 0; c < kTaps / kKc; ++c, ++g) {
-        const uint32_t stage = g % cqts::kStages, ph = (g / cqts::kStages) & 1u;
-        mbar_wait(a_full + stage, ph);
-        CQ_TRACE(icount, 7 + c);
-        tc_fence_after();
-        const uint32_t acol = tmem_base + stage * cqts::kAStageCols;
-#pragma unroll
-        for (int ks = 0; ks < kKc / 16; ++ks) {
-          const uint32_t ah = acol + (uint32_t)ks * 8u;
-          const uint32_t bo = w_base + (uint32_t)(((c * 3) * (kWPlane) + ks * 2 * (kN * 16)) >> 4);
-          umma_ts_bf16_x6(d, ah, ah + 32u, ah + 64u, bo, bo + (kWPlane >> 4), bo + 2 * (kWPlane >> 4), desc_hi32, idesc,
-                          (c | ks) ? 1u : 0u, leader);
-        }
-        umma_commit_pred(a_empty + stage, leader);
-      }
-      umma_commit_pred(tmem_full + buf, leader);
-      CQ_TRACE(icount, 11);
-      ++icount;
-    }
-  } else {
-    // ------------------------------ epilogue (warps 0..7), as in cqt_tc_kernel ------------------------------
-    const int quad = warp & 3, half = warp >> 2;
-    const int row = quad * 32 + lane;
-    const int nb = half ? 20 : 16, bin0 = half ? 16 : 0;
-    uint32_t ph_t[2] = {0, 0};
-    uint32_t icount = 0;
-    float* tile = s_tile + warp * (32 * kTilePitch);
-    for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
-      const int mt = it / kOctaves, o = it % kOctaves;
-      const int m = mt * kMTile + row;
-      const bool live = m < total_frames;
-      const int b = live ? m / kFrames : -1;
-      const uint32_t buf = icount & 1u;
-      mbar_wait(tmem_full + buf, ph_t[buf]);
-      ph_t[buf] ^= 1;
-      tc_fence_after();
-      if (warp == 0) CQ_TRACE(icount, 12);
-      const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (buf ? cqts::kAccCol1 : cqts::kAccCol0) + (uint32_t)(2 * bin0);
-      float vmin = INFINITY, vmax = -INFINITY;
-      const int g0 = (8 - o) * kBinsPerOctave - 15 + bin0;
-      uint32_t v[40];
-      tmem_ld32_nowait(taddr, reinterpret_cast<uint32_t(&)[32]>(v[0]));
-      if (half) {
-        uint32_t t8[8];
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                     : "=r"(t8[0]), "=r"(t8[1]), "=r"(t8[2]), "=r"(t8[3]), "=r"(t8[4]), "=r"(t8[5]), "=r"(t8[6]), "=r"(t8[7])
-                     : "r"(taddr + 32));
-#pragma unroll
-        for (int k = 0; k < 8; ++k) v[32 + k] = t8[k];
-      }
-      tmem_ld_wait();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(tmem_empty + buf);
-#pragma unroll
-      for (int j = 0; j < 20; ++j) {
-        if (j < nb) {
-          const int g = g0 + j;
-          float L = 0.f;
-          if (g >= 0) {
-            const float s = __ldg(a.scale + g);
-            const float re = __uint_as_float(v[2 * j]) * s, im = __uint_as_float(v[2 * j + 1]) * s;
-            L = __log2f(fmaf(re, re, im * im) + 1e-10f) * 3.0102999566398120f;
-            if (live) {
-              vmin = fminf(vmin, L);
-              vmax = fmaxf(vmax, L);
-            }
-          }
-          tile[lane * kTilePitch + j] = L;
-        }
-      }
-      __syncwarp();
-      {
-        const int m0 = mt * kMTile + quad * 32;
-        int rr = half ? lane / 20 : lane >> 4, jj = half ? lane - 20 * rr : lane & 15;
-        for (int i = 0; i < nb; ++i) {
-          if (m0 + rr < total_frames && g0 + jj >= 0) a.logmag[(size_t)(m0 + rr) * kCqtBins + g0 + jj] = tile[rr * kTilePitch + jj];
-          jj += 32;
-          if (half) {
-            rr += 1 + (jj >= 40);
-            jj -= jj >= 40 ? 40 : 20;
-          } else {
-            rr += 2;
-            jj -= 32;
-          }
-        }
-      }
-      __syncwarp();
-      const int b0 = __shfl_sync(0xffffffffu, b, 0);
-      const bool uniform = __all_sync(0xffffffffu, b == b0);
-      if (uniform) {
-        if (b0 >= 0) {
-#pragma unroll
-          for (int off = 16; off; off >>= 1) {
-            vmin = fminf(vmin, __shfl_xor_sync(0xffffffffu, vmin, off));
-            vmax = fmaxf(vmax, __shfl_xor_sync(0xffffffffu, vmax, off));
-          }
-          if (lane == 0 && vmin <= vmax) {
-            atomicMin(a.minmax + 2 * b0, float_to_ordered(vmin));
-            atomicMax(a.minmax + 2 * b0 + 1, float_to_ordered(vmax));
-          }
-        }
-      } else if (live && vmin <= vmax) {
-        atomicMin(a.minmax + 2 * b, float_to_ordered(vmin));
-        atomicMax(a.minmax + 2 * b + 1, float_to_ordered(vmax));
-      }
-      if (warp == 0) CQ_TRACE(icount, 13);
-      ++icount;
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == kMmaWarp) {
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
   }
 }
@@ -817,8 +392,7 @@ __global__ void minmax_init_kernel2(unsigned int* mm, int n) {
 }
 
 void cqt_tc_setup() {
-  cudaFuncSetAttribute(cqt_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cq::kSmemBytes);
-  cudaFuncSetAttribute(cqt_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cqts::kSmemBytes);
+  cudaFuncSetAttribute(cqt_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cq::kSmemBytes);
 }
 
 void launch_cqt_tc(const float* audio, const WinDesc* desc, const float* chain, const uint16_t* wtc, const float* scale,
@@ -846,19 +420,13 @@ void launch_cqt_tc(const float* audio, const WinDesc* desc, const float* chain, 
   a.n_mtiles = (n_windows * kFrames + cq::kMTile - 1) / cq::kMTile;
   const int n_items = a.n_mtiles * kOctaves;
   const int grid = n_items < n_sms ? n_items : n_sms;
-  // default: A operand in tensor memory (cqt_ts_kernel, 0.57 us/window); BP_B200_CQT_SS=1 selects the shared-memory operand
-  // kernel (0.67 us/window; same products in the same order, bit-identical output)
-  static const bool ts_form = getenv("BP_B200_CQT_SS") == nullptr;
-  if (ts_form)
-    cqt_ts_kernel<<<grid, cq::kThreads, cqts::kSmemBytes, st>>>(a);
-  else
-    cqt_tc_kernel<<<grid, cq::kThreads, cq::kSmemBytes, st>>>(a);
+  cqt_ts_kernel<<<grid, cq::kThreads, cq::kSmemBytes, st>>>(a);
 #ifdef BP_TC_TRACE
   if (tracing) {
     static long long h[64 * 16];
     cudaMemcpyAsync(h, d_trace, sizeof(h), cudaMemcpyDeviceToHost, st);
     cudaStreamSynchronize(st);
-    fprintf(stderr, "cqt_trace n_items %d grid %d (columns: item start, segment staged, stage acquired c0..c3, acc acquired, operands arrived c0..c3, MMAs issued, epilogue saw, epilogue done)\n", n_items, grid);
+    fprintf(stderr, "cqt_trace n_items %d grid %d (columns: 0 item start, 1 unused, 2-5 stage acquired c0..c3, 6 acc acquired, 7-10 operands arrived c0..c3, 11 MMAs issued, 12 epilogue saw, 13 epilogue done, 14-15 split done c2, c3)\n", n_items, grid);
     for (int i = 0; i < 64 && h[i * 16]; ++i) {
       fprintf(stderr, "item %2d (octave %d):", i, (i * grid) % 9);
       for (int e = 0; e < 16; ++e) fprintf(stderr, " %7lld", h[i * 16 + e] ? h[i * 16 + e] - h[0] : -1);

@@ -55,7 +55,6 @@
 //   warp 11     conv2 MMA issuer (A operand in tensor memory)
 //   warps 0-3, 4-7  epilogue, one warpgroup-like set of 4 warps (= the 4 TMEM lane quadrants) per accumulator slot:
 //               tcgen05.ld the accumulator columns, + bias, ReLU, split, tcgen05.st; then the conv2 sums as described above
-#include <cuda.h>  // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint)
 #include <cuda_bf16.h>
 
 #include <algorithm>
@@ -451,8 +450,6 @@ __global__ void lognorm_split_kernel(const float* __restrict__ y, const unsigned
 // The tensor-core kernel
 // ------------------------------------------------------------------------------------------------
 struct TcArgs {
-  CUtensorMap data_map;         // 4-D tensor map of `data`: (8 elements, rows_total, chunks8, 2 planes); box = one data tile
-  int use_tmap;                 // 0: the encoder was not available, the tile is fetched chunk by chunk with 1-D bulk copies
   const __nv_bfloat16* data;    // [2][chunks8][rows_total][8]
   const uint16_t* tiles;        // [n_tiles][8192 B]
   const uint16_t* b2;           // conv2 weight tiles (tc_build_b2), fused layers
@@ -894,14 +891,12 @@ __global__ void __launch_bounds__(tc::kThreads, 1) conv_tc_kernel(const __grid_c
       const size_t row = (size_t)mt * a.ms + a.row0;
       if (leader) {
         mbar_expect_tx(data_full, 2 * plane_bytes);
-        if (a.use_tmap) {  // one tensor-map TMA for the whole (planes x chunks x rows x 8 elements) tile
-          tma_load_4d(s_data, &a.data_map, 0, (int)row, 0, 0, data_full);
-        } else {
-          for (int p = 0; p < 2; ++p)
-            for (int c = 0; c < a.chunks8 - 1; ++c)
-              bulk_g2s(s_data + p * plane_bytes + c * lbo, a.data + p * plane_elems + ((size_t)c * a.rows_total + row) * 8,
-                       lbo, data_full);
-        }
+        // One 1-D bulk copy per plane and chunk: one 4-D tensor-map box measured 1.6 % slower (its innermost dimension is only
+        // 16 B, and a chunk of 2 080 B (contour: 130 rows x 16 B) cannot be split into 128-byte-aligned boxes).
+        for (int p = 0; p < 2; ++p)
+          for (int c = 0; c < a.chunks8 - 1; ++c)
+            bulk_g2s(s_data + p * plane_bytes + c * lbo, a.data + p * plane_elems + ((size_t)c * a.rows_total + row) * 8, lbo,
+                     data_full);
       }
       __syncwarp();
       ph_d ^= 1;
@@ -1300,38 +1295,6 @@ void launch_conv_tc(const __nv_bfloat16* data, const TcConvDev& dev, const TcOut
   a.g0 = sp.G0;
   const int n_items = a.n_mtiles * a.n_split;
   const int grid = n_items < n_sms ? n_items : n_sms;
-  {
-    // tensor map of the split input: dims (innermost first) 8 elements, rows, 8-bin chunks, hi / lo plane
-    using EncodeFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    static EncodeFn encode = [] {
-      void* fn = nullptr;
-      cudaDriverEntryPointQueryResult q;
-      if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) != cudaSuccess ||
-          q != cudaDriverEntryPointSuccess)
-        fn = nullptr;
-      return reinterpret_cast<EncodeFn>(fn);
-    }();
-    // The data tile can be fetched by ONE tensor-map TMA (cp.async.bulk.tensor.4d -> UTMALDG) or by 78 1-D bulk copies
-    // (one per plane and chunk).  Measured on the same B200 (tools/stage_times.py, A/B in one run): the tensor-map form is
-    // 1.6 % slower on the conv kernels (contour 0.990 vs 0.974, onset 1.390 vs 1.368 us/window) — its innermost box
-    // dimension is only 16 bytes, and one box is walked by one TMA pipeline while the bulk copies proceed in parallel
-    // (splitting the box is not possible: a chunk is 130 rows x 16 B = 2 080 B, not a multiple of the 128-byte shared-
-    // memory alignment a box needs).  Default = bulk copies; BP_B200_TMAP=1 selects the tensor map (GPU-tested).
-    a.use_tmap = 0;
-    static const bool want_tmap = getenv("BP_B200_TMAP") != nullptr;
-    if (encode && want_tmap) {
-      const cuuint64_t dims[4] = {8, (cuuint64_t)rows_stride, (cuuint64_t)sp.chunks8, 2};
-      const cuuint64_t strides[3] = {16, (cuuint64_t)rows_stride * 16, (cuuint64_t)sp.chunks8 * rows_stride * 16};
-      const cuuint32_t box[4] = {8, (cuuint32_t)a.data_rows, (cuuint32_t)(sp.chunks8 - 1), 2};
-      const cuuint32_t estr[4] = {1, 1, 1, 1};
-      if (encode(&a.data_map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<__nv_bfloat16*>(data), dims, strides, box, estr,
-                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS)
-        a.use_tmap = 1;
-    }
-  }
 #ifdef BP_TC_TRACE
   static long long* d_trace = nullptr;
   const bool tracing = getenv("BP_TC_TRACE") != nullptr;

@@ -106,14 +106,6 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, u
                "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar))
                : "memory");
 }
-// Tensor-map TMA: one 4-D box (cp.async.bulk.tensor -> UTMALDG) into shared memory, completion on an mbarrier
-__device__ __forceinline__ void tma_load_4d(void* smem_dst, const void* tmap, int c0, int c1, int c2, int c3, uint64_t* bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];" ::"r"(
-          smem_u32(smem_dst)),
-      "l"(tmap), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
 // expect_tx + bulk copy by the elected lane only (PTX predication): with warp-uniform operands the producer loop stays on
 // the uniform datapath (no per-step R2UR / elect loop around UBLKCP)
 __device__ __forceinline__ void bulk_g2s_expect_pred(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar,
@@ -172,34 +164,6 @@ __device__ __forceinline__ void umma_bf16_x3(uint32_t tmem_d, uint32_t a_hi_lo32
       "}\n" ::"r"(tmem_d),
       "r"(a_hi_lo32), "r"(a_lo_lo32), "r"(b_hi_lo32), "r"(b_lo_lo32), "r"(desc_hi32), "r"(idesc), "r"(accumulate),
       "r"(leader)
-      : "memory");
-}
-// The six products of a three-way split (a = h + m + l, b likewise): D (+)= Ah*Bh ; += Ah*Bm ; += Am*Bh ; += Ah*Bl ; += Al*Bh ; += Am*Bm,
-// issued by the elected lane only.  Descriptors as (low word, shared high word), see umma_bf16_x3.
-__device__ __forceinline__ void umma_bf16_x6(uint32_t tmem_d, uint32_t a_h, uint32_t a_m, uint32_t a_l, uint32_t b_h,
-                                             uint32_t b_m, uint32_t b_l, uint32_t desc_hi32, uint32_t idesc,
-                                             uint32_t accumulate, uint32_t leader) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p, q, t;\n\t"
-      ".reg .b64 dah, dam, dal, dbh, dbm, dbl;\n\t"
-      "setp.ne.b32 p, %9, 0;\n\t"
-      "setp.ne.b32 q, %10, 0;\n\t"
-      "setp.eq.b32 t, 0, 0;\n\t"
-      "mov.b64 dah, {%1, %7};\n\t"
-      "mov.b64 dam, {%2, %7};\n\t"
-      "mov.b64 dal, {%3, %7};\n\t"
-      "mov.b64 dbh, {%4, %7};\n\t"
-      "mov.b64 dbm, {%5, %7};\n\t"
-      "mov.b64 dbl, {%6, %7};\n\t"
-      "@q tcgen05.mma.cta_group::1.kind::f16 [%0], dah, dbh, %8, p;\n\t"
-      "@q tcgen05.mma.cta_group::1.kind::f16 [%0], dah, dbm, %8, t;\n\t"
-      "@q tcgen05.mma.cta_group::1.kind::f16 [%0], dam, dbh, %8, t;\n\t"
-      "@q tcgen05.mma.cta_group::1.kind::f16 [%0], dah, dbl, %8, t;\n\t"
-      "@q tcgen05.mma.cta_group::1.kind::f16 [%0], dal, dbh, %8, t;\n\t"
-      "@q tcgen05.mma.cta_group::1.kind::f16 [%0], dam, dbm, %8, t;\n\t"
-      "}\n" ::"r"(tmem_d),
-      "r"(a_h), "r"(a_m), "r"(a_l), "r"(b_h), "r"(b_m), "r"(b_l), "r"(desc_hi32), "r"(idesc), "r"(accumulate), "r"(leader)
       : "memory");
 }
 // Six products of a three-way split with the A operand in tensor memory (TS form): a_* are tensor-memory addresses (K = 16 ->
